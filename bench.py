@@ -240,6 +240,10 @@ def run_train(args, rank: int, world: int, local_rank: int, light: bool = False)
                       "steps": n_steps, "workload": f"c5: {desc}", "per_gpu": c}
     if light:
         return collective
+    # host copy now: the end-to-end steps below train further.  The last timed step's loss report, its (all-reduced)
+    # flat gradient and the parameters after its Adam update
+    outputs = {"grad": trainer.flat_grad.cpu().numpy(), "params": trainer.flat.cpu().numpy(),
+               **{k: np.float64(v) for k, v in rep_last.items() if not k.endswith("_size")}}
 
     # end to end: Trainer.train_step from host graphs + host labels, report read back every step
     targets = lab
@@ -260,6 +264,8 @@ def run_train(args, rank: int, world: int, local_rank: int, light: bool = False)
         if world > 1:
             dist.barrier()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     # breakdown of one resident step (synchronised, outside the timed loops)
     from chgnet_b200.engine import EV_A3_TO_GPA
     from chgnet_b200.trainer import loss_and_seeds
@@ -317,6 +323,21 @@ def run_train(args, rank: int, world: int, local_rank: int, light: bool = False)
         "last_report": rep_last, "breakdown": breakdown, "kernel_shares": shares}), flush=True)
     if world > 1:
         dist.barrier()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """--dump-outputs: what the timed path returned in its last step, one `<name>.npy` per array (float64 stays float64,
+    everything else is written as float32), so that two builds can be compared output for output on the same inputs."""
+    out = {k: np.asarray(v, dtype=np.float64 if np.asarray(v).dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_LIMIT_BYTES})")
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, f"{k}.npy"), a)
 
 
 def counts(graphs):
@@ -599,7 +620,7 @@ def infer_leg(model, graphs, dev, local_rank: int, world: int, steps: int, warmu
         flush()
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
-        step_resident()
+        last = step_resident()
         e.record()
         e.synchronize()
         elapsed_ms += s.elapsed_time(e)
@@ -607,6 +628,8 @@ def infer_leg(model, graphs, dev, local_rank: int, world: int, steps: int, warmu
     wall_ms = (time.perf_counter() - t_wall0) * 1e3
     launches = K.launches - launches0
     clocks = sampler.stop()
+    # host copy now: a replayed CUDA graph reuses its output tensors, and later legs replay it
+    outputs = {name: t.cpu().numpy() for name, t in zip(("energy", "force", "stress"), last)}
 
     # ---------------- end to end through the public API ----------------
     def step_e2e():
@@ -629,7 +652,7 @@ def infer_leg(model, graphs, dev, local_rank: int, world: int, steps: int, warmu
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     return {"ms_per_step": float(t[0].item()) / steps, "e2e_ms_per_step": float(t[1].item()) / steps, "launches": int(launches),
-            "clocks": clocks, "wall_ms": wall_ms, "h2d": h2d, "d2h": d2h, "preds": preds, "batch": batch}
+            "clocks": clocks, "wall_ms": wall_ms, "h2d": h2d, "d2h": d2h, "preds": preds, "batch": batch, "outputs": outputs}
 
 
 def md_leg(model, dev, steps: int = 20) -> dict:
@@ -786,6 +809,8 @@ def run_ours(args, rank: int, world: int, local_rank: int) -> None:
         if world > 1:
             dist.barrier()  # wait for rank 0's extra legs (roofline, shares, c4, CPU baseline)
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, leg["outputs"])
     # e2e breakdown (one synchronised pass, outside the timed loops)
     native = model._get_native()
     torch.cuda.synchronize()
@@ -967,7 +992,13 @@ def main() -> None:
     ap.add_argument("--no-md", action="store_true", help="skip the MD sub-leg of the c4 extra leg")
     ap.add_argument("--graph-replay", action="store_true", help="kernel-path leg: replay one captured CUDA graph of chg_forward per step")
     ap.add_argument("--scatter-only", action="store_true", help="run only the AtomConv scatter kernel timing (ncu target)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                    "(inference: energy, force, stress; c5: loss terms, grad, params); at N > 1, rank 0's share")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.scatter_only):
+        ap.error("--dump-outputs applies to the product arm's timed path (--impl ours, without --scatter-only)")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))

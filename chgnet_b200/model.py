@@ -783,8 +783,8 @@ class CHGNet(nn.Module):
     def load(cls, *, model_name: str = "0.3.0", use_device: str | None = None, check_cuda_mem: bool = False,
              verbose: bool = True):
         """Load a pretrained model (reference model.py:690-745).  Checkpoints are looked up in
-        $CHGNET_PRETRAINED_DIR, an installed ``chgnet`` package, /root/reference, then the
-        plain-array export under tests/golden (0.3.0 only)."""
+        $CHGNET_PRETRAINED_DIR, an installed ``chgnet`` package, then the plain-array exports
+        under tests/golden."""
         rel = _CHECKPOINTS.get(model_name)
         if rel is None:
             raise ValueError(f"Unknown {model_name=}")
@@ -797,7 +797,6 @@ class CHGNet(nn.Module):
                 roots.append(os.path.join(list(spec.submodule_search_locations)[0], "pretrained"))
         except (ImportError, ValueError):
             pass
-        roots.append("/root/reference/chgnet/pretrained")
         model = None
         for root in roots:
             if root and os.path.exists(os.path.join(root, rel)):
