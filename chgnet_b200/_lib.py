@@ -144,9 +144,9 @@ class CudaKernels:
                 raise ChgnetB200Error("kernel arguments must be contiguous CUDA tensors")
 
     def set_option(self, name: str, value: int) -> None:
-        """A/B switches (include/chgnet_b200.h): 'linear_impl' 0 FFMA | 1 tcgen05 | 2 tcgen05+TMA rows |
-        3 warp-specialised tcgen05 + TMA tensor maps (default),
-        'gated_impl' 3 fused warp-specialised tcgen05 message + aggregation (default) | 0 FFMA 4x8 | 1 tcgen05 | 2 FFMA 8x8."""
+        """The one run-time option (include/chgnet_b200.h): 'ws_min_rows', the row count from which AtomConv /
+        BondConv inference calls run the warp-specialised tcgen05 kernels instead of the FFMA kernels (default
+        4096; 0 runs them on any graph)."""
         if self.lib.chg_set_option(name.encode(), int(value)) != 0:
             raise ChgnetB200Error(self.lib.chg_last_error().decode())
 
@@ -213,7 +213,7 @@ class CudaKernels:
 
     def _fused_work(self, n_rows: int, device) -> Tensor:
         """Grow-only scratch of the fused message + aggregation kernels (strip partials; the message itself
-        for the unfused A/B implementations)."""
+        when a call below 'ws_min_rows' takes the unfused FFMA path)."""
         need = int(self.lib.chg_gated_fused_workspace_floats(int(n_rows)))
         ws = getattr(self, "_fws", None)
         if ws is None or ws.device != device or ws.numel() < need:

@@ -1,8 +1,7 @@
-// Library-level pieces of the C ABI: error string, version, launch counter.
+// Library-level pieces of the C ABI: error string, version, launch counter, the one run-time option.
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -11,6 +10,7 @@ namespace chg {
 namespace {
 thread_local char g_err[512] = "";
 std::atomic<int64_t> g_launches{0};
+std::atomic<int> g_ws_min_rows{4096};  // gated_common.cuh
 }  // namespace
 
 void set_error(const char* fmt, ...) {
@@ -32,68 +32,12 @@ int sm_count() {  // of the CURRENT device (cached per device ordinal)
   }
   return n;
 }
-}  // namespace chg
-
-namespace chg {
-namespace {
-// implementation switches.  Defaults follow the measured A/B (profiles/): the dense feature-mixing GEMM runs on
-// the warp-specialised tcgen05 kernel (linear_impl 3); the AtomConv / BondConv message + aggregation runs as the
-// fused warp-specialised tcgen05 kernel of gated_ws.cu (gated_impl 3) wherever the engine calls the fused entry
-// points; gated_impl 0..2 select the older unfused kernels (FFMA 4x8 / tcgen05 / FFMA 8x8) for A/B runs.
-std::atomic<int> g_linear_impl{-1}, g_gated_impl{-1}, g_wgrad_impl{-1}, g_ws_min_rows{-1}, g_segsum_unroll{-1}, g_segsum_s{-1};
-int env_default(const char* name, int dflt) {
-  const char* e = getenv(name);
-  if (e == nullptr || e[0] == 0) return dflt;
-  if (e[0] >= '0' && e[0] <= '9') return e[0] - '0';
-  return e[0] == 't' ? 1 : 0;
-}
-}  // namespace
-int linear_impl() {
-  int v = g_linear_impl.load();
-  if (v < 0) { v = env_default("CHG_LINEAR_IMPL", 3); g_linear_impl.store(v); }
-  return v;
-}
-int ws_min_rows() {
-  int v = g_ws_min_rows.load();
-  if (v < 0) {
-    const char* e = getenv("CHG_WS_MIN_ROWS");
-    v = (e != nullptr && e[0] != 0) ? atoi(e) : 4096;
-    if (v < 0) v = 0;
-    g_ws_min_rows.store(v);
-  }
-  return v;
-}
-int wgrad_impl() {
-  int v = g_wgrad_impl.load();
-  if (v < 0) { v = env_default("CHG_WGRAD_IMPL", 1); g_wgrad_impl.store(v); }
-  return v;
-}
-// segment_sum: input rows in flight per lane-group (4 or 8) and a forced number of lane-groups per output row (0 = heuristic)
-int segsum_unroll() {
-  int v = g_segsum_unroll.load();
-  if (v < 0) { v = env_default("CHG_SEGSUM_UNROLL", 4) == 8 ? 8 : 4; g_segsum_unroll.store(v); }
-  return v;
-}
-int segsum_force_s() {
-  int v = g_segsum_s.load();
-  if (v < 0) { v = env_default("CHG_SEGSUM_S", 0); if (v != 1 && v != 2 && v != 4 && v != 8) v = 0; g_segsum_s.store(v); }
-  return v;
-}
-int gated_impl() {
-  int v = g_gated_impl.load();
-  if (v < 0) { v = env_default("CHG_GATED_IMPL", 3); g_gated_impl.store(v); }
-  return v;
-}
+int ws_min_rows() { return g_ws_min_rows.load(); }
 }  // namespace chg
 
 extern "C" int chg_set_option(const char* name, int32_t value) {
   if (name == nullptr) return CHG_ERR_ARG;
-  if (strcmp(name, "linear_impl") == 0) { chg::g_linear_impl.store(value < 0 ? 0 : (value > 3 ? 3 : value)); return CHG_OK; }
-  if (strcmp(name, "gated_impl") == 0) { chg::g_gated_impl.store(value < 0 ? 0 : (value > 3 ? 3 : value)); return CHG_OK; }
   if (strcmp(name, "ws_min_rows") == 0) { chg::g_ws_min_rows.store(value < 0 ? 0 : value); return CHG_OK; }
-  if (strcmp(name, "segsum_unroll") == 0) { chg::g_segsum_unroll.store(value == 8 ? 8 : 4); return CHG_OK; }
-  if (strcmp(name, "segsum_s") == 0) { chg::g_segsum_s.store((value == 1 || value == 2 || value == 4 || value == 8) ? value : 0); return CHG_OK; }
-  if (strcmp(name, "wgrad_impl") == 0) { chg::g_wgrad_impl.store(value != 0 ? 1 : 0); return CHG_OK; }
   chg::set_error("chg_set_option: unknown option %s", name);
   return CHG_ERR_ARG;
 }

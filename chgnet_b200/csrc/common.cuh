@@ -11,10 +11,6 @@ namespace chg {
 void set_error(const char* fmt, ...);
 void count_launch();
 int sm_count();
-int linear_impl();  // 1 = tcgen05, 0 = FFMA
-int gated_impl();
-int segsum_unroll();   // 4 or 8 input rows in flight per lane-group of chg_segment_sum
-int segsum_force_s();  // 0 = heuristic
 
 #define CHG_CHECK_ARG(cond, msg)                \
   do {                                          \

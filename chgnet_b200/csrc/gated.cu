@@ -11,9 +11,10 @@
 // LayerNorm / SiLU / sigmoid / bond-weight smoothing / residual in the epilogue.
 //
 // This file is the FFMA implementation (64-row tiles in shared memory, register-tiled
-// GEMM; measured shared-memory-bandwidth bound, profiles/SUMMARY_r01.md).  gated_tc.cu
-// is the tcgen05 implementation of the same entry points; CHG_GATED_IMPL=ffma selects
-// this one.  One persistent CTA per resident slot; weights stay in shared memory.
+// GEMM; measured shared-memory-bandwidth bound, profiles/SUMMARY_r01.md).  The AtomConv /
+// BondConv reverse and fused message + aggregation entry points hand inference calls of at least
+// ws_min_rows() rows to the warp-specialised tcgen05 kernels of gated_ws.cu; everything
+// else runs here.  One persistent CTA per resident slot; weights stay in shared memory.
 //
 // Thread map: 256 threads = 16 (ty) x 16 (tx); a thread owns rows ty*4..+3 and, in
 // each 64-wide half (core | gate), columns tx*4..+3 — so core and gate of the same
@@ -359,349 +360,6 @@ __global__ void __launch_bounds__(NTHR, 2) gated_bwd_kernel(const BwdArgs a) {
   }
 }
 
-// =====================================================================================
-// AtomConv / BondConv, 8x8-tile variant (gated_impl = 2): 128-row tiles, 8x8 register tiles.
-//
-// ncu on the 4x8-tile kernels above showed them bound by shared-memory OPERAND DELIVERY, not by
-// the FMA pipe: every FMA needed 2 bytes from shared memory (an LDS.128 occupies the 128 B/clk
-// crossbar for 4 cycles even when it is a broadcast), i.e. at most 64 of 128 FMA lanes busy.
-// Here the warps are specialised per half of the block-diagonal product (warps 0-3 core, 4-7
-// gate) so that a thread's 8 rows x 8 columns share their A operand: (8 + 8) floats per 64 FMAs
-// = 1 byte per FMA.  The accumulators go back through the shared tile, and the epilogue runs in
-// the 16-lane-per-row layout (LayerNorm by shuffles, coalesced stores) as before.
-// Measured (B200, c4): 3-20 % SLOWER than the 4x8 kernels above — the extra tile round trip,
-// two more block barriers and the lower occupancy of the reverse kernel cost more than the
-// operand traffic saves; the default stays on the 4x8 kernels.
-// =====================================================================================
-constexpr int TM2 = 128;
-
-struct Smem2 {
-  static constexpr int W_OFF = 0;                    // fwd: W2^T [64][128]; bwd: W2 [128][64]
-  static constexpr int TILE_OFF = W_OFF + 64 * 128;  // [128][HS]
-  static constexpr int B2_OFF = TILE_OFF + TM2 * HS;
-  static constexpr int LN_OFF = B2_OFF + 128;
-  static constexpr int IDX_OFF = LN_OFF + 256;
-  static constexpr int TOTAL_BYTES = (IDX_OFF + 3 * TM2) * 4;
-};
-
-// acc[i][j] = sum_k T[row0+i][half*64 + k] * B(k, col(j)),  col(j) = (j<4 ? cg*4+j : 32+cg*4+(j-4))
-// B(k, c) at sB[k*ldb + c]
-__device__ __forceinline__ void gemm_half_8x8(float (&acc)[8][8], const float* __restrict__ sT,
-                                              const float* __restrict__ sB, int ldb, int row0, int cg) {
-#pragma unroll
-  for (int i = 0; i < 8; ++i)
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-#pragma unroll 2
-  for (int k2 = 0; k2 < 32; ++k2) {  // two k per step: A as 8-byte loads keeps 16 (not 32) A registers live
-    float2 a[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) a[i] = *reinterpret_cast<const float2*>(sT + (row0 + i) * HS + k2 * 2);
-#pragma unroll
-    for (int kk = 0; kk < 2; ++kk) {
-      const float4 b0 = lds4(sB + (k2 * 2 + kk) * ldb + cg * 4);
-      const float4 b1 = lds4(sB + (k2 * 2 + kk) * ldb + 32 + cg * 4);
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const float v = kk == 0 ? a[i].x : a[i].y;
-        acc[i][0] = fmaf(v, b0.x, acc[i][0]);
-        acc[i][1] = fmaf(v, b0.y, acc[i][1]);
-        acc[i][2] = fmaf(v, b0.z, acc[i][2]);
-        acc[i][3] = fmaf(v, b0.w, acc[i][3]);
-        acc[i][4] = fmaf(v, b1.x, acc[i][4]);
-        acc[i][5] = fmaf(v, b1.y, acc[i][5]);
-        acc[i][6] = fmaf(v, b1.z, acc[i][6]);
-        acc[i][7] = fmaf(v, b1.w, acc[i][7]);
-      }
-    }
-  }
-}
-
-// the product of the whole 128-row tile, in place: tile[:, half] <- tile[:, half] . B_half
-template <bool FWD>
-__device__ __forceinline__ void tile_gemm_inplace(float* s_tile, const float* s_w, int tid) {
-  const int half = tid >> 7, u = tid & 127;
-  const int cg = u & 7, row0 = (u >> 3) * 8;
-  // fwd: B(k, c) = W2^T[k][half*64 + c] (ld 128); bwd: B(k, c) = W2[half*64 + k][c] (ld 64)
-  const float* sB = FWD ? s_w + half * 64 : s_w + half * 64 * 64;
-  float acc[8][8];
-  gemm_half_8x8(acc, s_tile + half * 64, sB, FWD ? 128 : 64, row0, cg);
-  __syncthreads();  // every warp has finished reading the operand tile
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    float* dst = s_tile + (row0 + i) * HS + half * 64 + cg * 4;
-    sts4(dst, make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]));
-    sts4(dst + 32, make_float4(acc[i][4], acc[i][5], acc[i][6], acc[i][7]));
-  }
-  __syncthreads();
-}
-
-template <int MODE>
-__global__ void __launch_bounds__(NTHR, 2) gated2_fwd_kernel(const FwdArgs a) {
-  extern __shared__ __align__(16) float smem[];
-  float* s_w = smem + Smem2::W_OFF;
-  float* s_tile = smem + Smem2::TILE_OFF;
-  float* s_b2 = smem + Smem2::B2_OFF;
-  float* s_ln = smem + Smem2::LN_OFF;
-  int* s_idx = reinterpret_cast<int*>(smem + Smem2::IDX_OFF);
-
-  const int tid = threadIdx.x;
-  const int tx = tid & 15, ty = tid >> 4;  // 16 lanes per row, 16 row groups
-  const int c0 = tx * 4;
-  const bool use_ln = a.ln != nullptr;
-  copy_to_smem(s_w, a.w2t, 64 * 128, tid);
-  if (tid < 128) s_b2[tid] = a.b2[tid];
-  if (use_ln) s_ln[tid] = a.ln[tid];
-
-  const int n_tiles = (a.n_rows + TM2 - 1) / TM2;
-  for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-    const int base = tile * TM2;
-    __syncthreads();
-    if (tid < TM2) {
-      const int r = min(base + tid, a.n_rows - 1);
-      s_idx[tid] = a.idx0[r];
-      s_idx[TM2 + tid] = a.idx1[r];
-      s_idx[2 * TM2 + tid] = a.idx2[r];
-    }
-    __syncthreads();
-
-    // (a) gather + add the pre-activation rows, SiLU -> tile
-#pragma unroll 1
-    for (int it = 0; it < 2; ++it) {
-      const int r0 = it * 64 + ty * 4;
-      float acc[4][8];
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-      gather_pre<TM2>(acc, a.p_a, a.p_b, a.p_c, s_idx, base, a.n_rows, r0, c0);
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int g = base + r0 + i;
-        if (a.save_pre != nullptr && g < a.n_rows) {
-          stg4(a.save_pre + (size_t)g * 128 + c0, make_float4(acc[i][0], acc[i][1], acc[i][2], acc[i][3]));
-          stg4(a.save_pre + (size_t)g * 128 + 64 + c0, make_float4(acc[i][4], acc[i][5], acc[i][6], acc[i][7]));
-        }
-        sts4(s_tile + (r0 + i) * HS + c0,
-             make_float4(silu_f(acc[i][0]), silu_f(acc[i][1]), silu_f(acc[i][2]), silu_f(acc[i][3])));
-        sts4(s_tile + (r0 + i) * HS + 64 + c0,
-             make_float4(silu_f(acc[i][4]), silu_f(acc[i][5]), silu_f(acc[i][6]), silu_f(acc[i][7])));
-      }
-    }
-    __syncthreads();
-
-    // (b) second layer: tile <- tile . W2^T (per half)
-    tile_gemm_inplace<true>(s_tile, s_w, tid);
-
-    // (c) epilogue
-    float4 g1, b1, g2, b2v;
-    if (use_ln) {
-      g1 = lds4(s_ln + c0);
-      b1 = lds4(s_ln + 64 + c0);
-      g2 = lds4(s_ln + 128 + c0);
-      b2v = lds4(s_ln + 192 + c0);
-    }
-    const float4 bc = lds4(s_b2 + c0), bg = lds4(s_b2 + 64 + c0);
-#pragma unroll 1
-    for (int it = 0; it < 2; ++it) {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int row = it * 64 + ty * 4 + i;
-        const int g = base + row;
-        const bool valid = g < a.n_rows;
-        const float4 pc = lds4(s_tile + row * HS + c0) + bc;
-        const float4 pg = lds4(s_tile + row * HS + 64 + c0) + bg;
-        if (a.save_p != nullptr && valid) {
-          stg4(a.save_p + (size_t)g * 128 + c0, pc);
-          stg4(a.save_p + (size_t)g * 128 + 64 + c0, pg);
-        }
-        float y1[4] = {pc.x, pc.y, pc.z, pc.w};
-        float y2[4] = {pg.x, pg.y, pg.z, pg.w};
-        if (use_ln) {
-          float xh[4], rstd;
-          ln_stats(y1, xh, rstd);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) y1[j] = fmaf(xh[j], f4at(g1, j), f4at(b1, j));
-          ln_stats(y2, xh, rstd);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) y2[j] = fmaf(xh[j], f4at(g2, j), f4at(b2v, j));
-        }
-        float4 o;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) f4at(o, j) = silu_f(y1[j]) * sigmoid_f(y2[j]);
-        if (MODE == ATOM) {
-          o = o * ldg4(a.wgt + (size_t)s_idx[2 * TM2 + row] * 64 + c0);
-        } else {
-          o = o * ldg4(a.wgt + (size_t)s_idx[row] * 64 + c0) * ldg4(a.wgt + (size_t)s_idx[TM2 + row] * 64 + c0);
-        }
-        if (valid) stg4(a.out + (size_t)g * 64 + c0, o);
-      }
-    }
-  }
-}
-
-template <int MODE>
-__global__ void __launch_bounds__(NTHR, 2) gated2_bwd_kernel(const BwdArgs a) {
-  extern __shared__ __align__(16) float smem[];
-  float* s_w = smem + Smem2::W_OFF;  // W2 [128][64]
-  float* s_tile = smem + Smem2::TILE_OFF;
-  float* s_ln = smem + Smem2::LN_OFF;
-  int* s_idx = reinterpret_cast<int*>(smem + Smem2::IDX_OFF);
-
-  const int tid = threadIdx.x;
-  const int tx = tid & 15, ty = tid >> 4;
-  const int c0 = tx * 4;
-  const bool use_ln = a.ln != nullptr;
-  copy_to_smem(s_w, a.w2, 128 * 64, tid);
-  if (use_ln) s_ln[tid] = a.ln[tid];
-
-  const int n_tiles = (a.n_rows + TM2 - 1) / TM2;
-  for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-    const int base = tile * TM2;
-    __syncthreads();
-    if (tid < TM2) {
-      const int r = min(base + tid, a.n_rows - 1);
-      s_idx[tid] = a.idx0[r];
-      s_idx[TM2 + tid] = a.idx1[r];
-      if (MODE == ATOM) s_idx[2 * TM2 + tid] = a.idx2[r];
-    }
-    __syncthreads();
-
-    float4 g1, g2, b1, b2v;
-    if (use_ln) {
-      g1 = lds4(s_ln + c0);
-      b1 = lds4(s_ln + 64 + c0);
-      g2 = lds4(s_ln + 128 + c0);
-      b2v = lds4(s_ln + 192 + c0);
-    }
-    // (a) gate recompute, bond-weight gradients, LayerNorm reverse -> g_p -> tile
-#pragma unroll 1
-    for (int it = 0; it < 2; ++it) {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int row = it * 64 + ty * 4 + i;
-        const int g = base + row;
-        const bool valid = g < a.n_rows;
-        const int r = min(g, a.n_rows - 1);
-        const float4 pc4 = ldg4(a.save_p + (size_t)r * 128 + c0);
-        const float4 pg4 = ldg4(a.save_p + (size_t)r * 128 + 64 + c0);
-        float y1[4] = {pc4.x, pc4.y, pc4.z, pc4.w};
-        float y2[4] = {pg4.x, pg4.y, pg4.z, pg4.w};
-        float xh1[4], xh2[4], rstd1 = 1.f, rstd2 = 1.f;
-        if (use_ln) {
-          ln_stats(y1, xh1, rstd1);
-          ln_stats(y2, xh2, rstd2);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            y1[j] = fmaf(xh1[j], f4at(g1, j), f4at(b1, j));
-            y2[j] = fmaf(xh2[j], f4at(g2, j), f4at(b2v, j));
-          }
-        }
-        float s1[4], core[4], gate[4];
-        float4 o;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          s1[j] = sigmoid_f(y1[j]);
-          core[j] = y1[j] * s1[j];
-          gate[j] = sigmoid_f(y2[j]);
-          f4at(o, j) = core[j] * gate[j];
-        }
-        float4 go;
-        if (MODE == ATOM) {
-          const float4 gm = ldg4(a.g_in + (size_t)s_idx[row] * 64 + c0);
-          const float4 w = ldg4(a.wgt + (size_t)s_idx[2 * TM2 + row] * 64 + c0);
-          if (valid) stg4(a.g_w0 + (size_t)g * 64 + c0, gm * o);
-          go = gm * w;
-        } else {
-          const float4 gm = ldg4(a.g_in + (size_t)s_idx[row] * 64 + c0);
-          const float4 wi = ldg4(a.wgt + (size_t)s_idx[row] * 64 + c0);
-          const float4 wj = ldg4(a.wgt + (size_t)s_idx[TM2 + row] * 64 + c0);
-          const float4 gmo = gm * o;
-          if (valid) {
-            stg4(a.g_w0 + (size_t)g * 64 + c0, gmo * wj);
-            stg4(a.g_w1 + (size_t)g * 64 + c0, gmo * wi);
-          }
-          go = gm * wi * wj;
-        }
-        float gy1[4], gy2[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float gj = f4at(go, j);
-          gy1[j] = gj * gate[j] * (s1[j] * fmaf(y1[j], 1.f - s1[j], 1.f));
-          gy2[j] = gj * core[j] * gate[j] * (1.f - gate[j]);
-        }
-        if (use_ln) {
-          float gx[4], sa = 0.f, sb = 0.f;
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            gx[j] = gy1[j] * f4at(g1, j);
-            sa += gx[j];
-            sb = fmaf(gx[j], xh1[j], sb);
-          }
-          sa = sum16(sa) * (1.f / 64.f);
-          sb = sum16(sb) * (1.f / 64.f);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) gy1[j] = rstd1 * (gx[j] - sa - xh1[j] * sb);
-          sa = 0.f, sb = 0.f;
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            gx[j] = gy2[j] * f4at(g2, j);
-            sa += gx[j];
-            sb = fmaf(gx[j], xh2[j], sb);
-          }
-          sa = sum16(sa) * (1.f / 64.f);
-          sb = sum16(sb) * (1.f / 64.f);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) gy2[j] = rstd2 * (gx[j] - sa - xh2[j] * sb);
-        }
-        sts4(s_tile + row * HS + c0, make_float4(gy1[0], gy1[1], gy1[2], gy1[3]));
-        sts4(s_tile + row * HS + 64 + c0, make_float4(gy2[0], gy2[1], gy2[2], gy2[3]));
-      }
-    }
-    __syncthreads();
-
-    // (b) g_h = g_p . W2 (per half), in place
-    tile_gemm_inplace<false>(s_tile, s_w, tid);
-
-    // (c) g_pre = g_h * silu'(pre)
-#pragma unroll 1
-    for (int it = 0; it < 2; ++it) {
-      const int r0 = it * 64 + ty * 4;
-      float pre[4][8];
-      if (MODE == ATOM) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-#pragma unroll
-          for (int j = 0; j < 8; ++j) pre[i][j] = 0.f;
-        gather_pre<TM2>(pre, a.p_a, a.p_b, nullptr, s_idx, base, a.n_rows, r0, c0);
-      } else {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const int r = min(base + r0 + i, a.n_rows - 1);
-          const float4 vc = ldg4(a.save_pre + (size_t)r * 128 + c0);
-          const float4 vg = ldg4(a.save_pre + (size_t)r * 128 + 64 + c0);
-          pre[i][0] = vc.x; pre[i][1] = vc.y; pre[i][2] = vc.z; pre[i][3] = vc.w;
-          pre[i][4] = vg.x; pre[i][5] = vg.y; pre[i][6] = vg.z; pre[i][7] = vg.w;
-        }
-      }
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int g = base + r0 + i;
-        const float4 hc = lds4(s_tile + (r0 + i) * HS + c0);
-        const float4 hg = lds4(s_tile + (r0 + i) * HS + 64 + c0);
-        if (g < a.n_rows) {
-          stg4(a.g_pre + (size_t)g * 128 + c0,
-               make_float4(hc.x * dsilu_f(pre[i][0]), hc.y * dsilu_f(pre[i][1]), hc.z * dsilu_f(pre[i][2]),
-                           hc.w * dsilu_f(pre[i][3])));
-          stg4(a.g_pre + (size_t)g * 128 + 64 + c0,
-               make_float4(hg.x * dsilu_f(pre[i][4]), hg.y * dsilu_f(pre[i][5]), hg.z * dsilu_f(pre[i][6]),
-                           hg.w * dsilu_f(pre[i][7])));
-        }
-      }
-    }
-  }
-}
-
 template <int MODE>
 int launch_fwd(const FwdArgs& a, cudaStream_t stream) {
   if (a.n_rows == 0) return CHG_OK;
@@ -738,18 +396,6 @@ int launch_bwd(const BwdArgs& a, cudaStream_t stream) {
   return launch_bwd_t<MODE, false>(a, stream);
 }
 
-template <typename KernelT, typename ArgsT>
-int launch2(KernelT kernel, const ArgsT& a, int& slots, cudaStream_t stream) {
-  if (a.n_rows == 0) return CHG_OK;
-  if (slots == 0) {
-    CHG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem2::TOTAL_BYTES));
-    slots = resident_ctas(kernel, Smem2::TOTAL_BYTES);
-  }
-  const int n_tiles = (a.n_rows + TM2 - 1) / TM2;
-  kernel<<<min(n_tiles, slots), NTHR, Smem2::TOTAL_BYTES, stream>>>(a);
-  CHG_LAUNCH_END();
-}
-
 }  // namespace
 }  // namespace chg
 
@@ -764,12 +410,6 @@ extern "C" int chg_atom_conv_fwd(const float* pcn, const float* pe, const float*
   if (n_edges == 0) return CHG_OK;
   CHG_CHECK_ARG(pcn && pe && wag && center && nbr && d2u && w2t && b2 && msg, "null pointer");
   FwdArgs a{pcn, pe, nullptr, nullptr, wag, center, nbr, d2u, n_edges, w2t, b2, ln, msg, save_pre, save_p};
-  const bool train = save_pre != nullptr;  // training extras exist in the default implementation only
-  if (gated_impl() == 1 && !train) return atom_conv_fwd_tc(a, as_stream(stream));  // 3 (fused default) -> FFMA here
-  if (gated_impl() == 2 && !train) {  // 8x8-tile variant (measured slower end to end; kept for A/B)
-    static int slots = 0;
-    return launch2(gated2_fwd_kernel<ATOM>, a, slots, as_stream(stream));
-  }
   return launch_fwd<ATOM>(a, as_stream(stream));
 }
 
@@ -782,12 +422,7 @@ extern "C" int chg_atom_conv_bwd(const float* pcn, const float* pe, const float*
   CHG_CHECK_ARG(pcn && pe && wag && center && nbr && d2u && save_p && g_agg && w2 && g_pre && g_w, "null pointer");
   BwdArgs a{pcn, pe, wag, center, nbr, d2u, n_edges, nullptr, save_p, g_agg, w2, ln, g_pre, g_w, nullptr, g_p, g_ln};
   const bool train = g_p != nullptr || g_ln != nullptr;
-  if (gated_impl() == 3 && !train && n_edges >= ws_min_rows()) return atom_conv_bwd_ws(a, as_stream(stream));  // warp-specialised tcgen05 (default)
-  if (gated_impl() == 1 && !train) return atom_conv_bwd_tc(a, as_stream(stream));
-  if (gated_impl() == 2 && !train) {  // 8x8-tile variant (measured slower end to end; kept for A/B)
-    static int slots = 0;
-    return launch2(gated2_bwd_kernel<ATOM>, a, slots, as_stream(stream));
-  }
+  if (!train && n_edges >= ws_min_rows()) return atom_conv_bwd_ws(a, as_stream(stream));  // warp-specialised tcgen05
   return launch_bwd<ATOM>(a, as_stream(stream));
 }
 
@@ -799,11 +434,6 @@ extern "C" int chg_bond_conv_fwd(const float* pij, const float* px, const float*
   if (n_angles == 0) return CHG_OK;
   CHG_CHECK_ARG(pij && px && pa && wbg && ang_atom && ang_i && ang_j && w2t && b2 && upd, "null pointer");
   FwdArgs a{pij, px, pa, nullptr, wbg, ang_i, ang_j, ang_atom, n_angles, w2t, b2, ln, upd, save_pre, save_p};
-  if (gated_impl() == 1) return bond_conv_fwd_tc(a, as_stream(stream));
-  if (gated_impl() == 2) {  // 8x8-tile variant (measured slower end to end; kept for A/B)
-    static int slots = 0;
-    return launch2(gated2_fwd_kernel<BOND>, a, slots, as_stream(stream));
-  }
   return launch_fwd<BOND>(a, as_stream(stream));
 }
 
@@ -817,12 +447,7 @@ extern "C" int chg_bond_conv_bwd(const float* save_pre, const float* save_p, con
   BwdArgs a{nullptr, nullptr, wbg, ang_i, ang_j, nullptr, n_angles, save_pre, save_p, g_agg, w2, ln,
             g_pre, gw_i, gw_j, g_p, g_ln};
   const bool train = g_p != nullptr || g_ln != nullptr;
-  if (gated_impl() == 3 && !train && n_angles >= ws_min_rows()) return bond_conv_bwd_ws(a, as_stream(stream));  // warp-specialised tcgen05 (default)
-  if (gated_impl() == 1 && !train) return bond_conv_bwd_tc(a, as_stream(stream));
-  if (gated_impl() == 2 && !train) {  // 8x8-tile variant (measured slower end to end; kept for A/B)
-    static int slots = 0;
-    return launch2(gated2_bwd_kernel<BOND>, a, slots, as_stream(stream));
-  }
+  if (!train && n_angles >= ws_min_rows()) return bond_conv_bwd_ws(a, as_stream(stream));  // warp-specialised tcgen05
   return launch_bwd<BOND>(a, as_stream(stream));
 }
 

@@ -1,4 +1,4 @@
-// Shared pieces of the gated-MLP kernels (FFMA: gated.cu, tcgen05: gated_tc.cu).
+// Shared pieces of the gated-MLP kernels (FFMA: gated.cu, gated_2nd.cu; warp-specialised tcgen05: gated_ws.cu).
 #pragma once
 #include "common.cuh"
 
@@ -9,7 +9,7 @@ constexpr int HS = 132;    // smem stride of a 128-wide row
 constexpr float LN_EPS = 1e-5f;
 }  // namespace gated
 // below this many rows the warp-specialised tcgen05 kernels hand the call to the FFMA kernels (launch-bound regime);
-// chg_set_option("ws_min_rows", n) / env CHG_WS_MIN_ROWS, default 4096 (abi.cu)
+// default 4096; chg_set_option("ws_min_rows", n) changes it (abi.cu), e.g. to run the tcgen05 kernels on small test graphs
 int ws_min_rows();
 namespace gated {
 
@@ -148,12 +148,6 @@ inline int resident_ctas(KernelT kernel, int smem_bytes) {
 }
 
 #endif
-
-// entry points of the tcgen05 implementation (gated_tc.cu)
-int atom_conv_fwd_tc(const FwdArgs& a, cudaStream_t stream);
-int bond_conv_fwd_tc(const FwdArgs& a, cudaStream_t stream);
-int atom_conv_bwd_tc(const BwdArgs& a, cudaStream_t stream);
-int bond_conv_bwd_tc(const BwdArgs& a, cudaStream_t stream);
 
 // warp-specialised tcgen05 reverse kernels (gated_ws.cu): same outputs as gated_bwd_kernel<MODE, false>
 int atom_conv_bwd_ws(const BwdArgs& a, cudaStream_t stream);

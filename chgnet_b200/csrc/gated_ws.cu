@@ -40,16 +40,7 @@ constexpr int TR = 128;          // rows per tile
 constexpr int HALF_BYTES = TR * 64 * 4;
 constexpr int IMG_BYTES = 64 * 64 * 4;
 constexpr int STRIP = 16;        // rows per reduction strip (one half-warp)
-#ifndef CHG_WS_REGSPLIT
-// 1: setmaxnreg in the forward kernel - 20 warps launched with 96 registers, then 144 for the producer warps (24 instead of 12
-// independent 16-byte gathers in flight per thread), 72 for the epilogue warps, 40 for the MMA warp's warpgroup (3 of its 4 warps
-// exist only to donate registers; the pool of a CTA is what it was launched with).  Measured on B200 (c3): AtomConv 1.53 -> 1.47 ms,
-// BondConv 1.55 -> 1.51 ms per step, i.e. the gathers' memory-level parallelism is NOT what bounds the kernel: left off.
-#define CHG_WS_REGSPLIT 0
-#endif
-constexpr int PB = CHG_WS_REGSPLIT ? 8 : 4;  // rows gathered per producer batch (x 3-4 loads each in flight)
-// register pool of the CTA = what it was launched with: 20 warps x 96; after the reallocation 8 x 72 + 8 x 144 + 4 x 40 = 1888 <= 1920
-constexpr int WS_FWD_THREADS = CHG_WS_REGSPLIT ? 640 : WS_THREADS;
+constexpr int PB = 4;            // rows gathered per producer batch (x 3-4 loads each in flight)
 
 struct WsSmem {
   static constexpr int IMG_OFF = 0;                          // Bc_hi, Bc_lo, Bg_hi, Bg_lo
@@ -167,7 +158,7 @@ __device__ __forceinline__ void epilogue_half(uint32_t d_addr, const float* s_b2
 }
 
 template <int MODE>
-__global__ void __launch_bounds__(WS_FWD_THREADS, 1) gated_ws_fwd_kernel(const FusedArgs a) {
+__global__ void __launch_bounds__(WS_THREADS, 1) gated_ws_fwd_kernel(const FusedArgs a) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* s_img = smem_raw + WsSmem::IMG_OFF;
   uint8_t* s_hs = smem_raw + WsSmem::HS_OFF;
@@ -208,11 +199,6 @@ __global__ void __launch_bounds__(WS_FWD_THREADS, 1) gated_ws_fwd_kernel(const F
 
   if (warp >= 8 && warp < 16) {
     // ============================ producer groups (gather -> SiLU -> A operand) ============================
-#if CHG_WS_REGSPLIT
-    // the gathers are what the kernel waits for: take registers from the epilogue warps (which give up 24 each) so that a
-    // producer thread keeps 24 instead of 12 independent 16-byte loads in flight
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 144;");
-#endif
     const int half = (warp - 8) >> 2;            // 0: core columns, 1: gate columns
     const int gt = tid - 256 - half * 128;       // 0..127 inside the group; also this thread's tile row / TMEM lane
     const int tx = gt & 15, ty = gt >> 4;        // 16 lanes per row, 8 rows per pass
@@ -284,10 +270,7 @@ __global__ void __launch_bounds__(WS_FWD_THREADS, 1) gated_ws_fwd_kernel(const F
       mbar_arrive(&bars.a_full[half]);
     }
   } else if (warp >= 16) {
-    // ============================ MMA issuer (warp 16; warps 17-19 only donate registers) ============================
-#if CHG_WS_REGSPLIT
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 40;");
-#endif
+    // ============================ MMA issuer (warp 16) ============================
     if (warp == 16 && lane == 0) {
       const uint32_t idesc = tc::idesc_tf32(128, 64);
       const uint32_t img = tc::smem_u32(s_img);
@@ -317,9 +300,6 @@ __global__ void __launch_bounds__(WS_FWD_THREADS, 1) gated_ws_fwd_kernel(const F
     }
   } else if (warp < 8) {
     // ============================ epilogue: warps 0-3 core half, warps 4-7 gate half ============================
-#if CHG_WS_REGSPLIT
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 72;");
-#endif
     const int eh = warp >> 2;        // 0: core, 1: gate
     const int t = tid & 127;         // tile row == TMEM lane
     const uint32_t lane_sel = (uint32_t)((warp & 3) * 32) << 16;
@@ -444,7 +424,7 @@ int launch_fused(const FusedArgs& a, cudaStream_t stream) {
       attr_set = true;
     }
     const int n_tiles = (a.n_rows + TR - 1) / TR;
-    gated_ws_fwd_kernel<MODE><<<min(n_tiles, sm_count()), WS_FWD_THREADS, WsSmem::TOTAL, stream>>>(a);
+    gated_ws_fwd_kernel<MODE><<<min(n_tiles, sm_count()), WS_THREADS, WsSmem::TOTAL, stream>>>(a);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {
       set_error("gated_ws_fwd_kernel: launch failed: %s", cudaGetErrorString(e));
@@ -494,10 +474,10 @@ extern "C" int chg_atom_conv_fused(const float* pcn, const float* pe, const floa
   CHG_CHECK_ARG(ptr_c && agg, "null pointer");
   CHG_CHECK_ARG(n_edges == 0 || (pcn && pe && wag && center && nbr && d2u && w2t && b2 && work), "null pointer");
   // tiny inputs (a few tiles) are launch-bound: the persistent tcgen05 kernel's fixed cost (weight images, TMEM) loses there
-  if (gated_impl() == 3 && n_edges >= ws_min_rows())
+  if (n_edges >= ws_min_rows())
     return gated::atom_conv_fused_ws(pcn, pe, wag, center, nbr, d2u, ptr_c, n_edges, n_atoms, w2t, b2, ln, agg, save_p, work,
                                      as_stream(stream));
-  // A/B implementations 0..2: the unfused pair (message kernel -> segmented sum), the message in `work`
+  // the unfused pair (FFMA message kernel -> segmented sum), the message in `work`
   const int rc = chg_atom_conv_fwd(pcn, pe, wag, center, nbr, d2u, n_edges, w2t, b2, ln, work, save_p, nullptr, stream);
   if (rc != CHG_OK) return rc;
   return chg_segment_sum(work, 64, nullptr, ptr_c, n_atoms, n_edges, 0, agg, 64, stream);
@@ -512,7 +492,7 @@ extern "C" int chg_bond_conv_fused(const float* pij, const float* px, const floa
   if (n_slots == 0) return CHG_OK;
   CHG_CHECK_ARG(ptr_i && agg, "null pointer");
   CHG_CHECK_ARG(n_angles == 0 || (pij && px && pa && wbg && ang_atom && ang_i && ang_j && w2t && b2 && work), "null pointer");
-  if (gated_impl() == 3 && n_angles >= ws_min_rows())
+  if (n_angles >= ws_min_rows())
     return gated::bond_conv_fused_ws(pij, px, pa, wbg, ang_atom, ang_i, ang_j, ptr_i, n_angles, n_slots, w2t, b2, ln, agg,
                                      save_pre, save_p, work, as_stream(stream));
   const int rc = chg_bond_conv_fwd(pij, px, pa, wbg, ang_atom, ang_i, ang_j, n_angles, w2t, b2, ln, work, save_pre, save_p, stream);

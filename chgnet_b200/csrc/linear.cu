@@ -126,8 +126,6 @@ int launch_linear(const float* x, const int32_t* x_rows, int m, int k, const flo
 
 int linear_tc(const float* x, const int32_t* x_rows, int m, int k, const float* wt, const float* bias,
               const float* residual, const int32_t* y_rows, int n_out, float* y, cudaStream_t stream);
-int linear_tma(const float* x, const int32_t* x_rows, int m, int k, const float* wt, const float* bias,
-               const float* residual, const int32_t* y_rows, int n_out, float* y, cudaStream_t stream);
 int linear_ws(const float* x, int m, int k, const float* wt, const float* bias, const float* residual, int n_out,
               float* y, cudaStream_t stream);
 
@@ -143,18 +141,15 @@ extern "C" int chg_linear(const float* x, const int32_t* x_rows, int32_t m, int3
   CHG_CHECK_ARG(n_out > 0 && n_out % 64 == 0, "n_out must be a positive multiple of 64");
   if (m == 0) return CHG_OK;
   CHG_CHECK_ARG(x && wt && y, "null pointer");
-  // tcgen05 paths: 1 = register-staged kernel (default: fastest over the whole step), 2 = TMA-fed
-  // kernel (k <= 128; wins only on the largest calls)
-  if (linear_impl() == 2 && k <= 128)
-    return linear_tma(x, x_rows, m, k, wt, bias, residual, y_rows, n_out, y, as_stream(stream));
-  // below ~4k rows the tensor-core kernel's fixed cost (operand images, TMEM allocation) is not
-  // amortised: the FFMA kernel is faster there (tools/linear_ab.py)
-  if (linear_impl() == 3 && m >= 4096 && x_rows == nullptr && y_rows == nullptr) {  // warp-specialised + TMA maps
-    const int rc = linear_ws(x, m, k, wt, bias, residual, n_out, y, as_stream(stream));
-    if (rc <= 0) return rc;  // rc == 1: not applicable, fall through
-  }
-  if (linear_impl() >= 1 && m >= 4096)
+  // below ~4k rows the tensor-core kernels' fixed cost (operand images, TMEM allocation) is not amortised: the FFMA
+  // kernel is faster there
+  if (m >= 4096) {
+    if (x_rows == nullptr && y_rows == nullptr) {  // warp-specialised, fed by 2-D TMA tensor maps
+      const int rc = linear_ws(x, m, k, wt, bias, residual, n_out, y, as_stream(stream));
+      if (rc <= 0) return rc;  // rc == 1: not applicable (k = 256, or no tensor map for these operands)
+    }
     return linear_tc(x, x_rows, m, k, wt, bias, residual, y_rows, n_out, y, as_stream(stream));
+  }
   if (n_out % 128 == 0 && k <= 128)
     return launch_linear<128>(x, x_rows, m, k, wt, bias, residual, y_rows, n_out, y, as_stream(stream));
   return launch_linear<64>(x, x_rows, m, k, wt, bias, residual, y_rows, n_out, y, as_stream(stream));

@@ -18,7 +18,7 @@
 namespace chg {
 namespace {
 
-template <int W, int S, int U>
+template <int W, int S>
 __global__ void __launch_bounds__(256)
 segment_sum_kernel(const float* __restrict__ data, const int32_t* __restrict__ perm,
                    const int32_t* __restrict__ ptr, int n_rows, int accumulate, float* out, int out_ld) {
@@ -41,20 +41,6 @@ segment_sum_kernel(const float* __restrict__ data, const int32_t* __restrict__ p
       const float* base = data + (size_t)sub * 4;
       int k = beg;
       if (perm == nullptr) {
-        if (U == 8) {  // eight rows in flight per lane-group; the same additions in the same order as the 4-row loop
-          for (; k + 7 * S < end; k += 8 * S) {
-            const float4 v0 = ldg4(base + (size_t)(k + 0 * S) * W);
-            const float4 v1 = ldg4(base + (size_t)(k + 1 * S) * W);
-            const float4 v2 = ldg4(base + (size_t)(k + 2 * S) * W);
-            const float4 v3 = ldg4(base + (size_t)(k + 3 * S) * W);
-            const float4 v4 = ldg4(base + (size_t)(k + 4 * S) * W);
-            const float4 v5 = ldg4(base + (size_t)(k + 5 * S) * W);
-            const float4 v6 = ldg4(base + (size_t)(k + 6 * S) * W);
-            const float4 v7 = ldg4(base + (size_t)(k + 7 * S) * W);
-            a0 = a0 + v0; a1 = a1 + v1; a2 = a2 + v2; a3 = a3 + v3;
-            a0 = a0 + v4; a1 = a1 + v5; a2 = a2 + v6; a3 = a3 + v7;
-          }
-        }
         for (; k + 3 * S < end; k += 4 * S) {
           const float4 v0 = ldg4(base + (size_t)(k + 0 * S) * W);
           const float4 v1 = ldg4(base + (size_t)(k + 1 * S) * W);
@@ -64,22 +50,6 @@ segment_sum_kernel(const float* __restrict__ data, const int32_t* __restrict__ p
         }
         for (; k < end; k += S) a0 = a0 + ldg4(base + (size_t)k * W);
       } else {
-        if (U == 8) {
-          for (; k + 7 * S < end; k += 8 * S) {
-            const int i0 = perm[k], i1 = perm[k + S], i2 = perm[k + 2 * S], i3 = perm[k + 3 * S];
-            const int i4 = perm[k + 4 * S], i5 = perm[k + 5 * S], i6 = perm[k + 6 * S], i7 = perm[k + 7 * S];
-            const float4 v0 = ldg4(base + (size_t)i0 * W);
-            const float4 v1 = ldg4(base + (size_t)i1 * W);
-            const float4 v2 = ldg4(base + (size_t)i2 * W);
-            const float4 v3 = ldg4(base + (size_t)i3 * W);
-            const float4 v4 = ldg4(base + (size_t)i4 * W);
-            const float4 v5 = ldg4(base + (size_t)i5 * W);
-            const float4 v6 = ldg4(base + (size_t)i6 * W);
-            const float4 v7 = ldg4(base + (size_t)i7 * W);
-            a0 = a0 + v0; a1 = a1 + v1; a2 = a2 + v2; a3 = a3 + v3;
-            a0 = a0 + v4; a1 = a1 + v5; a2 = a2 + v6; a3 = a3 + v7;
-          }
-        }
         for (; k + 3 * S < end; k += 4 * S) {
           const int i0 = perm[k], i1 = perm[k + S], i2 = perm[k + 2 * S], i3 = perm[k + 3 * S];
           const float4 v0 = ldg4(base + (size_t)i0 * W);
@@ -110,13 +80,17 @@ segment_sum_kernel(const float* __restrict__ data, const int32_t* __restrict__ p
   }
 }
 
-template <int W, int S, int U>
-void launch_segsum(const float* data, const int32_t* perm, const int32_t* ptr, int n_rows, int accumulate,
+template <int W>
+void launch_segsum(int S, const float* data, const int32_t* perm, const int32_t* ptr, int n_rows, int accumulate,
                    float* out, int out_ld, cudaStream_t stream) {
-  constexpr int ROWS = (256 / (W / 4)) / S;
-  const int n_pass = (n_rows + ROWS - 1) / ROWS;
+  const int rows = (256 / (W / 4)) / S;
+  const int n_pass = (n_rows + rows - 1) / rows;
   const int blocks = max(1, min(n_pass, sm_count() * 8));
-  segment_sum_kernel<W, S, U><<<blocks, 256, 0, stream>>>(data, perm, ptr, n_rows, accumulate, out, out_ld);
+  const auto kernel = S == 1   ? segment_sum_kernel<W, 1>
+                      : S == 2 ? segment_sum_kernel<W, 2>
+                      : S == 4 ? segment_sum_kernel<W, 4>
+                               : segment_sum_kernel<W, 8>;
+  kernel<<<blocks, 256, 0, stream>>>(data, perm, ptr, n_rows, accumulate, out, out_ld);
 }
 
 // dst[i] = src[idx[i]] (gather) or dst[idx[i]] = src[i] (scatter); rows of `width` floats
@@ -176,19 +150,9 @@ extern "C" int chg_segment_sum(const float* data, int32_t width, const int32_t* 
   // long segments with one lane-group each leave a latency-bound tail (the last, longest segments stream with 4 loads
   // in flight): two groups per row even when that takes more than one wave (c3: 67.5 -> 64.3 us, c4: 75.7 -> 71.8 us)
   if (S == 1 && avg >= 32) S = 2;
-  if (segsum_force_s() > 0) S = segsum_force_s();
-  const bool u8 = segsum_unroll() == 8;
-  cudaStream_t st = as_stream(stream);
-#define CHG_SEG(W_, S_)                                                              \
-  do {                                                                               \
-    if (u8) launch_segsum<W_, S_, 8>(data, perm, ptr, n_rows, accumulate, out, out_ld, st); \
-    else launch_segsum<W_, S_, 4>(data, perm, ptr, n_rows, accumulate, out, out_ld, st);    \
-  } while (0)
-  if (width == 64) {
-    if (S == 1) CHG_SEG(64, 1); else if (S == 2) CHG_SEG(64, 2); else if (S == 4) CHG_SEG(64, 4); else CHG_SEG(64, 8);
-  } else {
-    if (S == 1) CHG_SEG(128, 1); else if (S == 2) CHG_SEG(128, 2); else if (S == 4) CHG_SEG(128, 4); else CHG_SEG(128, 8);
-  }
-#undef CHG_SEG
+  if (width == 64)
+    launch_segsum<64>(S, data, perm, ptr, n_rows, accumulate, out, out_ld, as_stream(stream));
+  else
+    launch_segsum<128>(S, data, perm, ptr, n_rows, accumulate, out, out_ld, as_stream(stream));
   CHG_LAUNCH_END();
 }

@@ -488,7 +488,6 @@ void wgrad_reduce_launch(const float* partial, const float* cs_partial, int n_ch
 int wgrad_tc(const float* x, const float* x2, int ldx, const int32_t* x_rows, int x_silu, const float* g, int ldg,
              const int32_t* g_rows, int m, int n_out, float* out, int ldo, float* colsum, float* workspace, int max_chunks,
              cudaStream_t stream);  // wgrad_tc.cu: returns 1 when it does not take the call
-int wgrad_impl();  // abi.cu: 1 = tcgen05 (default), 0 = FFMA
 }  // namespace chg
 
 using namespace chg;
@@ -508,12 +507,11 @@ extern "C" int chg_wgrad(const float* x, const float* x2, int32_t ldx, const int
   CHG_CHECK_ARG(ldx >= 64 && ldx % 4 == 0 && ldg >= n_out && ldg % 4 == 0 && ldo >= n_out, "bad leading dimension");
   CHG_CHECK_ARG((((uintptr_t)x | (uintptr_t)x2 | (uintptr_t)g | (uintptr_t)workspace) & 15) == 0,
                 "x, x2, g, workspace must be 16-byte aligned");
-  if (wgrad_impl() == 1) {  // tensor cores (3xTF32) for the large reductions; same partial buffer, same fp64 second pass
-    const int64_t cap = std::min<int64_t>(WG_MAX_CHUNKS, (int64_t)sm_count() * 2 * std::max(1, 256 / n_out));
-    const int rc = wgrad_tc(x, x2, ldx, x_rows, x_silu, g, ldg, g_rows, m, n_out, out, ldo, colsum, workspace, (int)cap,
-                            as_stream(stream));
-    if (rc != 1) return rc;
-  }
+  // tensor cores (3xTF32) for the large reductions; same partial buffer, same fp64 second pass
+  const int64_t cap = std::min<int64_t>(WG_MAX_CHUNKS, (int64_t)sm_count() * 2 * std::max(1, 256 / n_out));
+  const int rc = wgrad_tc(x, x2, ldx, x_rows, x_silu, g, ldg, g_rows, m, n_out, out, ldo, colsum, workspace, (int)cap,
+                          as_stream(stream));
+  if (rc != 1) return rc;  // 1: not taken (small reduction): the FFMA kernel below
   const int steps = (m + WG_ROWS - 1) / WG_ROWS;
   // narrow outputs get more row chunks (more CTAs per SM in flight: the kernel is latency bound)
   const int n_chunks = max(1, min(min(steps, sm_count() * 2 * max(1, 256 / n_out)), WG_MAX_CHUNKS));

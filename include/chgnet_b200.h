@@ -44,20 +44,12 @@ const char* chg_last_error(void);
 int chg_abi_version(void);
 /* number of kernel launches issued by this library since load (host counter) */
 int64_t chg_launch_count(void);
-/* implementation switches for A/B measurements (same results, same ABI):
- *   "linear_impl": 0 FFMA, 1 tcgen05 register-staged, 2 tcgen05 + TMA row copies,
- *                  3 warp-specialised tcgen05 fed by 2-D TMA tensor maps (default; calls with
- *                    row indirection or k = 256 use 1)
- *   "gated_impl" : 3 fused warp-specialised tcgen05 message + aggregation (default; chg_*_conv_fused),
- *                  0 FFMA 4x8 tiles, 1 tcgen05 (un-pipelined), 2 FFMA 8x8 tiles (all unfused; with 3 the
- *                  unfused entry points chg_*_conv_fwd / _bwd run the FFMA 4x8 kernels)
- *   "ws_min_rows": calls with fewer rows than this (default 4096) run the FFMA kernels even with gated_impl 3
- *                  (launch-bound regime: the persistent tcgen05 kernels' fixed cost loses on a few tiles)
- *   "wgrad_impl" : 1 tcgen05 3xTF32 for reductions over >= 4096 rows (default; csrc/wgrad_tc.cu), 0 FFMA
- *   "segsum_unroll": 4 (default) or 8 input rows in flight per lane-group of chg_segment_sum (identical results)
- *   "segsum_s"   : 0 (default: chosen from the mean segment length) or 1 / 2 / 4 / 8 lane-groups per output row
- * (env CHG_LINEAR_IMPL / CHG_GATED_IMPL = 0..3, CHG_WGRAD_IMPL = 0..1, CHG_WS_MIN_ROWS, CHG_SEGSUM_UNROLL, CHG_SEGSUM_S set
- * the defaults; CHG_PACK_THREADS = worker threads of the host packers / many-structure builder, default min(16, cores)). */
+/* run-time option (returns CHG_ERR_ARG for any other name):
+ *   "ws_min_rows": AtomConv / BondConv inference calls with at least this many rows (default 4096) run the
+ *                  warp-specialised tcgen05 kernels, smaller ones the FFMA kernels (launch-bound regime: the
+ *                  persistent tcgen05 kernels' fixed cost loses on a few tiles).  Tests set 0 to run the tcgen05
+ *                  kernels on small graphs.
+ * (env CHG_PACK_THREADS = worker threads of the host packers / many-structure builder, default min(16, cores)). */
 int chg_set_option(const char* name, int32_t value);
 
 /* ---- K0: atom embedding.  x[i] = emb[z[i]-1]   (model.py:432-434, encoders.py:32) */
@@ -150,8 +142,8 @@ int chg_segment_sum(const float* data, int32_t width, const int32_t* perm,
  * second-layer products as 3xTF32 on the tensor cores, LayerNorm / SiLU x sigmoid, and the segmented sum inside the
  * CTA (the [rows][64] message never reaches HBM), followed by a small stitch kernel for segments that span
  * 16-row strips (fixed order: deterministic).  save_p / save_pre [rows][128] may be NULL (no reverse pass).
- * `work`: caller scratch of chg_gated_fused_workspace_floats(rows) floats.  With gated_impl 0..2 the same entry
- * points run the unfused pair chg_*_conv_fwd -> chg_segment_sum (A/B).                                        */
+ * `work`: caller scratch of chg_gated_fused_workspace_floats(rows) floats.  Calls with fewer rows than
+ * "ws_min_rows" (chg_set_option) run the unfused FFMA pair chg_*_conv_fwd -> chg_segment_sum instead.         */
 int64_t chg_gated_fused_workspace_floats(int32_t n_rows);
 int chg_atom_conv_fused(const float* pcn, const float* pe, const float* wag, const int32_t* center,
                         const int32_t* nbr, const int32_t* d2u, const int32_t* ptr_c, int32_t n_edges,

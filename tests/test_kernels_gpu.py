@@ -38,17 +38,14 @@ def recorded(weights030):
     return _record(weights030, graphs, need_grad=True, need_magmom=True, need_atom_fea=True, need_crystal_fea=True)
 
 
-@pytest.mark.parametrize("linear_impl,gated_impl", [(3, 3), (3, 0), (1, 0), (0, 1), (2, 2)],
-                         ids=["defaults: linear=tcgen05-ws,gated=fused-tcgen05-ws", "linear=tcgen05-ws,gated=ffma4x8",
-                              "linear=tcgen05,gated=ffma4x8", "linear=ffma,gated=tcgen05", "linear=tcgen05+tma,gated=ffma8x8"])
-def test_every_kernel_matches_its_spec(recorded, linear_impl, gated_impl):
-    """Both implementations of every entry point (tcgen05 3xTF32 and FFMA) against the spec."""
+@pytest.mark.parametrize("ws_min_rows", [0, 4096], ids=["tcgen05-ws-forced", "defaults-ffma"])
+def test_every_kernel_matches_its_spec(recorded, ws_min_rows):
+    """Both implementations of the AtomConv / BondConv entry points (warp-specialised tcgen05 3xTF32 and FFMA), and
+    every other kernel, against the spec."""
     from chgnet_b200._lib import CudaKernels
 
     K = CudaKernels()
-    K.set_option("linear_impl", linear_impl)
-    K.set_option("gated_impl", gated_impl)
-    K.set_option("ws_min_rows", 0)  # the recorded graphs are small: run the tcgen05 kernels on them anyway
+    K.set_option("ws_min_rows", ws_min_rows)  # the recorded graphs are small: 0 runs the tcgen05 kernels on them anyway
     try:
         seen = {}
         for name, snap, outs in recorded:
@@ -61,8 +58,6 @@ def test_every_kernel_matches_its_spec(recorded, linear_impl, gated_impl):
         assert set(seen) == __import__("kernel_replay").INFER_KERNELS, sorted(seen)
         print({k: f"{v:.2e}" for k, v in seen.items()})
     finally:
-        K.set_option("linear_impl", 3)
-        K.set_option("gated_impl", 3)
         K.set_option("ws_min_rows", 4096)
 
 
@@ -132,35 +127,40 @@ def test_loss_terms_and_adam_match_torch():
         assert float((p - ref.detach()).abs().max()) < 2e-6
 
 
-@pytest.mark.parametrize("impl", [3, 2, 1, 0], ids=["tcgen05-ws", "tcgen05+tma", "tcgen05", "ffma"])
-def test_linear_large_ragged_calls(impl):
-    """chg_linear at the sizes where the tensor-core kernels are dispatched (m >= 4096): ragged
-    last tile, every (k, n) the model uses, bias / residual / in-place residual, against fp64."""
+@pytest.mark.parametrize("m", [1, 63, 4095, 4096, 5001, 70001], ids=lambda m: f"m={m}")
+def test_linear_ragged_calls(m):
+    """chg_linear on both sides of the 4096-row switch from the FFMA kernels (NT = 64 and 128) to the tensor-core
+    kernels: ragged last tile, every (k, n) the model uses, bias / residual / in-place residual, and a gathered call
+    (x_rows, as the engine makes for the bond-graph rows), against fp64."""
     from chgnet_b200._lib import CudaKernels
 
     K = CudaKernels()
-    K.set_option("linear_impl", impl)
     g = torch.Generator(device="cuda").manual_seed(5)
-    try:
-        for m in (4096, 5001, 70001):
-            for k, n in ((64, 128), (64, 256), (128, 64), (64, 64), (64, 192), (128, 128), (256, 64)):
-                for has_bias, res_mode in ((True, "none"), (False, "separate"), (True, "inplace")):
-                    x = torch.randn(m, k, device="cuda", generator=g)
-                    wt = torch.randn(k, n, device="cuda", generator=g) / k ** 0.5
-                    bias = torch.randn(n, device="cuda", generator=g) if has_bias else None
-                    res = torch.randn(m, n, device="cuda", generator=g) if res_mode != "none" else None
-                    want = x.double() @ wt.double()
-                    if bias is not None:
-                        want += bias.double()
-                    if res is not None:
-                        want += res.double()
-                    y = res if res_mode == "inplace" else torch.full((m, n), float("nan"), device="cuda")
-                    K.linear(x, wt, bias, res, y, None, None)
-                    torch.cuda.synchronize()
-                    err = float((y.double() - want).abs().max())
-                    assert err < 5e-5, (impl, m, k, n, has_bias, res_mode, err)
-    finally:
-        K.set_option("linear_impl", 3)
+    for k, n in ((64, 128), (64, 256), (128, 64), (64, 64), (64, 192), (128, 128), (256, 64)):
+        for has_bias, res_mode in ((True, "none"), (False, "separate"), (True, "inplace")):
+            x = torch.randn(m, k, device="cuda", generator=g)
+            wt = torch.randn(k, n, device="cuda", generator=g) / k ** 0.5
+            bias = torch.randn(n, device="cuda", generator=g) if has_bias else None
+            res = torch.randn(m, n, device="cuda", generator=g) if res_mode != "none" else None
+            want = x.double() @ wt.double()
+            if bias is not None:
+                want += bias.double()
+            if res is not None:
+                want += res.double()
+            y = res if res_mode == "inplace" else torch.full((m, n), float("nan"), device="cuda")
+            K.linear(x, wt, bias, res, y, None, None)
+            torch.cuda.synchronize()
+            err = float((y.double() - want).abs().max())
+            assert err < 5e-5, (m, k, n, has_bias, res_mode, err)
+    x = torch.randn(2 * m + 7, 64, device="cuda", generator=g)
+    rows = torch.randint(0, x.shape[0], (m,), device="cuda", generator=g, dtype=torch.int32)
+    wt = torch.randn(64, 256, device="cuda", generator=g) / 8
+    bias = torch.randn(256, device="cuda", generator=g)
+    y = torch.full((m, 256), float("nan"), device="cuda")
+    K.linear(x, wt, bias, None, y, rows)
+    torch.cuda.synchronize()
+    err = float((y.double() - (x.double()[rows.long()] @ wt.double() + bias.double())).abs().max())
+    assert err < 5e-5, (m, "x_rows", err)
 
 
 def test_kernels_without_layernorm_and_small_basis(weights030):
@@ -222,53 +222,50 @@ def test_bad_arguments_are_reported():
         K.linear(torch.zeros(4, 64), torch.zeros(64, 64), None, None, torch.zeros(4, 64))  # CPU tensors
 
 
-@pytest.mark.parametrize("wgrad_impl", [1, 0], ids=["tcgen05", "ffma"])
-def test_wgrad_large_reduction_matches_fp64(wgrad_impl):
-    """chg_wgrad at the sizes where the tensor-core kernel (csrc/wgrad_tc.cu, 3xTF32) takes over (>= 4096 rows): plain,
-    SiLU'd and tangent activations, row gathers on either operand, strided operands, column sums - against fp64."""
+@pytest.mark.parametrize("m", [20011, 4095], ids=lambda m: f"m={m}")
+def test_wgrad_large_reduction_matches_fp64(m):
+    """chg_wgrad on both sides of the 4096-row switch from the FFMA kernel to the tensor-core kernel (csrc/wgrad_tc.cu,
+    3xTF32): plain, SiLU'd and tangent activations, row gathers on either operand, strided operands, column sums -
+    against fp64."""
     from chgnet_b200._lib import CudaKernels
 
     K = CudaKernels()
-    K.set_option("wgrad_impl", wgrad_impl)
-    try:
-        gen = torch.Generator(device="cuda").manual_seed(5)
-        m = 20011  # not a multiple of the 64-row stage
-        xs = torch.randn(m, 128, device="cuda", generator=gen)
-        x2 = torch.randn(m, 128, device="cuda", generator=gen)
-        gs = torch.randn(m, 256, device="cuda", generator=gen)
-        perm = torch.randperm(m, device="cuda", generator=gen).int()
-        sub = perm[:9000].contiguous()
-        silu, dsilu = torch.nn.functional.silu, (lambda t: torch.sigmoid(t) * (1 + t * (1 - torch.sigmoid(t))))
-        cases = [
-            dict(x=xs[:, :64], g=gs[:, :128], n=128),
-            dict(x=xs[:, 64:], g=gs[:, 64:128], n=64, x_silu=True, colsum=True),
-            dict(x=xs[:, :64], g=gs[:, 128:], n=128, x2=x2[:, :64]),
-            dict(x=xs[:, :64], g=gs[:, :128], n=128, x_rows=sub, colsum=True),
-            dict(x=xs[:, 64:], g=gs[:, :64], n=64, g_rows=sub),
-        ]
-        for c in cases:
-            n = c["n"]
-            out = torch.empty(64, n, device="cuda")
-            cs = torch.empty(n, device="cuda") if c.get("colsum") else None
-            K.wgrad(c["x"], c["g"], out, cs, c.get("x_rows"), c.get("g_rows"), c.get("x_silu", False), c.get("x2"))
-            torch.cuda.synchronize()
-            xr = c["x"].double() if c.get("x_rows") is None else c["x"].double()[c["x_rows"].long()]
-            gr = c["g"].double() if c.get("g_rows") is None else c["g"].double()[c["g_rows"].long()]
-            if c.get("g_rows") is not None and c.get("x_rows") is None:
-                xr = xr[: gr.shape[0]]
-            if c.get("x_rows") is not None and c.get("g_rows") is None:
-                gr = gr[: xr.shape[0]]
-            act = xr
-            if c.get("x_silu"):
-                act = silu(xr)
-            if c.get("x2") is not None:
-                act = dsilu(xr) * c["x2"].double()
-            want = act.T @ gr
-            scale = float(want.abs().max())
-            err = float((out.double() - want).abs().max())
-            assert err < 3e-5 * scale + 1e-5, (wgrad_impl, c.keys(), err, scale)
-            if cs is not None:
-                wc = gr.sum(dim=0)
-                assert float((cs.double() - wc).abs().max()) < 3e-5 * float(wc.abs().max()) + 1e-4
-    finally:
-        K.set_option("wgrad_impl", 1)
+    gen = torch.Generator(device="cuda").manual_seed(5)
+    # neither size is a multiple of the 64-row stage
+    xs = torch.randn(m, 128, device="cuda", generator=gen)
+    x2 = torch.randn(m, 128, device="cuda", generator=gen)
+    gs = torch.randn(m, 256, device="cuda", generator=gen)
+    perm = torch.randperm(m, device="cuda", generator=gen).int()
+    sub = perm[: 9000 * m // 20011].contiguous()
+    silu, dsilu = torch.nn.functional.silu, (lambda t: torch.sigmoid(t) * (1 + t * (1 - torch.sigmoid(t))))
+    cases = [
+        dict(x=xs[:, :64], g=gs[:, :128], n=128),
+        dict(x=xs[:, 64:], g=gs[:, 64:128], n=64, x_silu=True, colsum=True),
+        dict(x=xs[:, :64], g=gs[:, 128:], n=128, x2=x2[:, :64]),
+        dict(x=xs[:, :64], g=gs[:, :128], n=128, x_rows=sub, colsum=True),
+        dict(x=xs[:, 64:], g=gs[:, :64], n=64, g_rows=sub),
+    ]
+    for c in cases:
+        n = c["n"]
+        out = torch.empty(64, n, device="cuda")
+        cs = torch.empty(n, device="cuda") if c.get("colsum") else None
+        K.wgrad(c["x"], c["g"], out, cs, c.get("x_rows"), c.get("g_rows"), c.get("x_silu", False), c.get("x2"))
+        torch.cuda.synchronize()
+        xr = c["x"].double() if c.get("x_rows") is None else c["x"].double()[c["x_rows"].long()]
+        gr = c["g"].double() if c.get("g_rows") is None else c["g"].double()[c["g_rows"].long()]
+        if c.get("g_rows") is not None and c.get("x_rows") is None:
+            xr = xr[: gr.shape[0]]
+        if c.get("x_rows") is not None and c.get("g_rows") is None:
+            gr = gr[: xr.shape[0]]
+        act = xr
+        if c.get("x_silu"):
+            act = silu(xr)
+        if c.get("x2") is not None:
+            act = dsilu(xr) * c["x2"].double()
+        want = act.T @ gr
+        scale = float(want.abs().max())
+        err = float((out.double() - want).abs().max())
+        assert err < 3e-5 * scale + 1e-5, (m, c.keys(), err, scale)
+        if cs is not None:
+            wc = gr.sum(dim=0)
+            assert float((cs.double() - wc).abs().max()) < 3e-5 * float(wc.abs().max()) + 1e-4

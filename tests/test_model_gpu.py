@@ -47,21 +47,17 @@ def test_limno2_known_answers(model, limno2_graph, golden):
     print({k: f"{_maxabs(out[k], golden[f'limno2.oracle64.{k}']):.2e}" for k in TOL})
 
 
-@pytest.mark.parametrize("linear_impl,gated_impl", [(1, 1), (0, 0), (3, 3)], ids=["all-tcgen05", "all-ffma", "defaults"])
-def test_limno2_parity_for_every_implementation(model, limno2_graph, golden, linear_impl, gated_impl):
+@pytest.mark.parametrize("ws_min_rows", [0, 4096], ids=["tcgen05-ws-forced", "defaults-ffma"])
+def test_limno2_parity_for_every_implementation(model, limno2_graph, golden, ws_min_rows):
     from chgnet_b200._lib import CudaKernels
 
     K = CudaKernels()
-    K.set_option("linear_impl", linear_impl)
-    K.set_option("gated_impl", gated_impl)
-    K.set_option("ws_min_rows", 0)  # 8-atom cell: force the tcgen05 kernels where gated_impl asks for them
+    K.set_option("ws_min_rows", ws_min_rows)  # 8-atom cell: 0 forces the warp-specialised tcgen05 kernels
     try:
         out = model.predict_graph(limno2_graph)
         for k, tol in TOL.items():
             assert _maxabs(out[k], golden[f"limno2.oracle64.{k}"]) < tol, k
     finally:
-        K.set_option("linear_impl", 3)
-        K.set_option("gated_impl", 3)
         K.set_option("ws_min_rows", 4096)
 
 

@@ -24,6 +24,4 @@ timeout 900 ncu --set full --clock-control none --import-source on -k regex:gate
   -o gpurun_out/prof_gated_${TAG} -f python bench.py --workload c4 --steps 1 --warmup 1 --no-cpu-baseline > gpurun_out/ncu_gated.log 2>&1
 timeout 900 ncu --set full --clock-control none --import-source on -k regex:linear_tc -s 30 -c 4 \
   -o gpurun_out/prof_linear_${TAG} -f python bench.py --workload c4 --steps 1 --warmup 1 --no-cpu-baseline > gpurun_out/ncu_linear.log 2>&1
-CHG_GATED_IMPL=tc timeout 900 ncu --set full --clock-control none --import-source on -k regex:gated_.*tc -s 8 -c 4 \
-  -o gpurun_out/prof_gatedtc_${TAG} -f python bench.py --workload c4 --steps 1 --warmup 1 --no-cpu-baseline > gpurun_out/ncu_gatedtc.log 2>&1
 ls -la gpurun_out | tail -30

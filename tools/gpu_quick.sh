@@ -1,8 +1,7 @@
 #!/bin/bash
-# quick iteration: linear A/B (tc), GPU tests, bench c2 + c4 without the CPU baseline leg
+# quick iteration: GPU tests, bench c2 + c4 without the CPU baseline leg
 mkdir -p gpurun_out
 TAG=${1:-q}
-# (linear A/B: tools/gpu_tc.sh)
 timeout 900 python -m pytest tests -m gpu -x -q 2>&1 | tail -6
 for wl in c2 c4; do
   timeout 600 python bench.py --workload $wl --steps 10 --warmup 3 --no-cpu-baseline > gpurun_out/bench_${wl}_${TAG}.json 2> gpurun_out/bench_${wl}_${TAG}.err
