@@ -35,12 +35,12 @@ def _maxabs(a, b):
     return float(np.max(np.abs(np.asarray(a, dtype=np.float64) - np.asarray(b, dtype=np.float64))))
 
 
-def _compare(model, weights, graphs, batch_size, oracle_batch, label):
+def _compare(model, weights, graphs, batch_size, oracle_batch, label, args=None):
     from oracle import chgnet_oracle as orc
 
     preds = model.predict_graph(graphs, task="efsm", batch_size=batch_size)
     # the fp64 oracle runs its (stock torch) ops on the GPU here: same checker, seconds instead of minutes
-    ref = orc.predict_graph(weights, graphs, "efsm", batch_size=oracle_batch, dtype=torch.float64, device="cuda")
+    ref = orc.predict_graph(weights, graphs, "efsm", batch_size=oracle_batch, dtype=torch.float64, device="cuda", args=args)
     if not isinstance(preds, list):
         preds, ref = [preds], [ref]
     worst = {k: max(_maxabs(p[k], r[k]) for p, r in zip(preds, ref)) for k in TOL}
@@ -67,6 +67,35 @@ def test_c4_shaped_supercell_vs_fp64_oracle(model, weights030, supercell):
     g = graphgen.make_crystal_graph(z, frac, lat)
     (p,) = _compare(model, weights030, [g], 1, 1, f"LiMnO2 {supercell} = {len(z)} atoms")
     assert np.abs(p["f"].sum(axis=0)).max() < 1e-3  # translation invariance at size
+
+
+def test_v020_checkpoint_at_tcgen05_size_vs_fp64_oracle(monkeypatch):
+    """The 0.2.0 checkpoint (no gMLP LayerNorm, 5 A cutoff) on a 216-atom LiMnO2 supercell: every AtomConv and
+    BondConv call has at least 4096 rows, so the default dispatch runs the tcgen05 kernels without LayerNorm, forward
+    and reverse.  The oracle runs with the checkpoint's weights and arguments (the keys
+    oracle/make_golden_checkpoints.py passes it)."""
+    import json
+
+    from chgnet_b200.model import CHGNet
+
+    monkeypatch.setenv("CHGNET_PRETRAINED_DIR", "/nonexistent")  # use the committed plain-array export
+    model = CHGNet.load(model_name="0.2.0", use_device="cuda", verbose=False)
+    with np.load(os.path.join(GOLD, "chgnet_0.2.0_weights.npz")) as f:
+        weights = {k: f[k] for k in f.files if k != "__model_args__"}
+        margs = json.loads(str(f["__model_args__"]))
+    keys = ("num_radial", "num_angular", "gMLP_norm", "readout_norm", "mlp_out_bias", "cutoff_coeff",
+            "atom_graph_cutoff", "bond_graph_cutoff", "n_conv", "is_intensive")
+    args = {k: margs[k] for k in keys if k in margs}
+    args["atom_graph_cutoff"], args["bond_graph_cutoff"] = float(args["atom_graph_cutoff"]), float(args["bond_graph_cutoff"])
+    assert args["gMLP_norm"] is None and args["atom_graph_cutoff"] == 5.0
+    z, frac, lat = graphgen.limno2_structure((3, 3, 3), 0.02, 4002)
+    g = graphgen.make_crystal_graph(z, frac, lat, atom_graph_cutoff=args["atom_graph_cutoff"],
+                                    bond_graph_cutoff=args["bond_graph_cutoff"])
+    # rows of the AtomConv calls (directed edges) and the BondConv calls (angles) vs the default ws_min_rows
+    n_edges, n_angles = int(g.atom_graph.shape[0]), int(g.bond_graph.shape[0])
+    assert min(n_edges, n_angles) >= 4096, (n_edges, n_angles)
+    _compare(model, weights, [g], 1, 1, f"0.2.0, LiMnO2 (3, 3, 3) = {len(z)} atoms, {n_edges} edges, {n_angles} angles",
+             args=args)
 
 
 def test_c5_slice_parameter_gradients_efsm(model, weights030):
