@@ -41,6 +41,11 @@ SIGNATURES: dict[str, list] = {
     "chg_readout": [P, P, P, I, P, P, P, P, I, P, F, P, P, P, P, P, P, P],
     "chg_magmom": [P, I, P, F, P, P],
     "chg_force_virial": [P, P, P, P, P, P, P, P, P, P, I, P, P, P],
+    # Berendsen NVT / NPT with the cell on the device (dynamics_device.DeviceMD)
+    "chg_md_partial_blocks": [I],
+    "chg_md_cell_step": [P, P, P, I, P, P, I, P],
+    "chg_md_kick_drift_cell": [P, P, P, P, I, ctypes.c_double, P, P, P, P, P, I, P],
+    "chg_md_kick_partials": [P, P, P, I, ctypes.c_double, P, P],
     # training
     "chg_wgrad": [P, P, I, P, I, P, I, P, I, I, P, I, P, P, P],
     "chg_colsum": [P, I, P, I, P, I, I, P, P],

@@ -71,6 +71,16 @@ class Atoms:
     def get_masses(self):
         return ATOMIC_MASSES[self.numbers - 1]
 
+    def get_volume(self) -> float:
+        return abs(float(np.linalg.det(self.cell)))
+
+    def set_cell(self, cell, scale_atoms: bool = False) -> None:
+        """New cell; ``scale_atoms=True`` keeps the fractional coordinates (ase's ``Atoms.set_cell``)."""
+        cell = np.asarray(cell, dtype=np.float64).reshape(3, 3)
+        if scale_atoms:
+            self.positions = (self.positions @ np.linalg.inv(self.cell)) @ cell
+        self.cell = cell.copy()
+
     def __len__(self) -> int:
         return len(self.numbers)
 
@@ -182,6 +192,132 @@ class VelocityVerlet:
             log.append({"step": self.nsteps, "e_pot": self.potential_energy(), "e_kin": self.kinetic_energy(),
                         "temperature": self.temperature()})
         return log
+
+
+def berendsen_lambda(temperature: float, target: float, dt_over_taut: float) -> float:
+    """Velocity scale of ASE's ``NVTBerendsen.scale_velocities``: sqrt(1 + (T0 / T - 1) dt / tau_t) clamped to
+    [0.9, 1.1]; 1.1 at T = 0 (ASE divides by zero there and clamps the infinity)."""
+    if temperature == 0.0:
+        return 1.1
+    a = 1.0 + (target / temperature - 1.0) * dt_over_taut
+    return 0.9 if a <= 0.81 else min(max(float(np.sqrt(a)), 0.9), 1.1)
+
+
+class NVTBerendsen(VelocityVerlet):
+    """Berendsen NVT on the host (ASE's ``NVTBerendsen``, the reference's default ensemble, dynamics.py:595-609),
+    the checker of ``DeviceMD(ensemble="nvt")``.  One step, with F (and the stress) of the previous call:
+
+    1. thermostat: T = K_tr / (3 N k_B), v <- lambda v (``berendsen_lambda``);
+    2. barostat (the NPT subclasses): P_a = -sigma_aa + K_aa / V, then the cell is scaled with the atoms;
+    3. v <- v + dt/2 F/m;  4. ``fix_com``: v_i <- v_i - mean(m v) / m_i;  5. x <- x + dt v;
+    6. one ``calculate`` (forces, stress);  7. v <- v + dt/2 F/m.
+
+    ``temperature`` in K, ``pressure`` / ``bulk_modulus`` in GPa, ``timestep`` / ``taut`` / ``taup`` in fs.  Any object
+    with ``calculate(atoms, task=...)`` and ``results`` {"energy", "forces", "stress" (eV/A^3)} can drive it."""
+
+    barostat: str | None = None
+
+    def __init__(self, atoms, calculator, timestep: float = 2.0, temperature: float = 300.0, taut: float | None = None,
+                 fix_com: bool = True, task: PredTask | None = None) -> None:
+        self.fix_com = fix_com
+        self.target_temperature = float(temperature)
+        self.dt_over_taut = (timestep * FS) / ((100.0 * timestep if taut is None else taut) * FS)
+        super().__init__(atoms, calculator, timestep=timestep, task=task or ("efs" if self.barostat else "ef"))
+        self.stress = self._stress()
+
+    def _stress(self) -> np.ndarray | None:
+        if self.barostat is None:
+            return None
+        return np.asarray(self.calc.results["stress"], dtype=np.float64).reshape(3, 3)
+
+    def set_target(self, temperature: float | None = None, pressure: float | None = None) -> None:
+        if temperature is not None:
+            self.target_temperature = float(temperature)
+        if pressure is not None:
+            self.target_pressure = float(pressure) * GPA
+
+    def scale_cell(self) -> None:
+        """The barostat (NPT subclasses)."""
+
+    def step(self) -> None:
+        atoms, m = self.atoms, self.atoms.get_masses()[:, None]
+        self.last_lambda = berendsen_lambda(self.temperature(), self.target_temperature, self.dt_over_taut)
+        atoms.velocities = self.last_lambda * atoms.velocities
+        self.scale_cell()
+        v = atoms.velocities + 0.5 * self.dt * self.forces / m
+        if self.fix_com:
+            p = m * v
+            v = (p - p.sum(axis=0) / len(p)) / m
+        atoms.velocities = v
+        atoms.positions = atoms.positions + self.dt * v
+        self.calc.calculate(atoms, task=self.task)
+        self.forces = np.asarray(self.calc.results["forces"], dtype=np.float64)
+        self.stress = self._stress()
+        atoms.velocities = atoms.velocities + 0.5 * self.dt * self.forces / m
+        self.nsteps += 1
+
+    def pressure_components(self) -> np.ndarray:
+        """P_a = -sigma_aa + K_aa / V in eV/A^3 (ase's ``get_stress(include_ideal_gas=True)``, diagonal, negated)."""
+        m = self.atoms.get_masses()[:, None]
+        k = (m * self.atoms.velocities**2).sum(axis=0)
+        return -np.diag(self.stress) + k / self.atoms.get_volume()
+
+    def run(self, steps: int) -> list[dict]:
+        log = []
+        for _ in range(steps):
+            self.step()
+            entry = {"step": self.nsteps, "e_pot": self.potential_energy(), "e_kin": self.kinetic_energy(),
+                     "temperature": self.temperature()}
+            if self.barostat is not None:
+                entry["volume"] = self.atoms.get_volume()
+                entry["pressure"] = float(self.pressure_components().mean()) / GPA
+            log.append(entry)
+        return log
+
+
+class Inhomogeneous_NPTBerendsen(NVTBerendsen):  # noqa: N801  (ASE's name)
+    """Berendsen NPT with one scale per lattice vector (ASE's ``Inhomogeneous_NPTBerendsen``, dynamics.py:671-691):
+    mu_a = 1 - dt beta / (3 tau_p) (P0 - P_a) mask_a, row a of the cell times mu_a, so the angles are kept.
+    The step is the one of :class:`NVTBerendsen`; the forces of the previous call are used after the cell is scaled
+    (one model call per step, as ``DeviceMD``; ASE calls the model again there)."""
+
+    barostat = "inhomogeneous"
+
+    def __init__(self, atoms, calculator, timestep: float = 2.0, temperature: float = 300.0, pressure: float = 1.01325e-4,
+                 taut: float | None = None, taup: float | None = None, bulk_modulus: float | None = None,
+                 fix_com: bool = True, mask=(1, 1, 1), task: PredTask | None = None) -> None:
+        if bulk_modulus is None:
+            raise ValueError("npt needs bulk_modulus (GPa)")
+        self.target_pressure = float(pressure) * GPA
+        beta = 1.0 / (float(bulk_modulus) * GPA)
+        self.taupscl = (timestep * FS) / ((1000.0 * timestep if taup is None else taup) * FS) * beta / 3.0
+        self.mask = np.asarray(mask, dtype=np.float64)
+        super().__init__(atoms, calculator, timestep=timestep, temperature=temperature, taut=taut, fix_com=fix_com, task=task)
+
+    def mu(self) -> np.ndarray:
+        return 1.0 - self.taupscl * (self.target_pressure - self.pressure_components()) * self.mask
+
+    def scale_cell(self) -> None:
+        self.atoms.set_cell(self.mu()[:, None] * self.atoms.cell, scale_atoms=True)
+
+
+class NPTBerendsen(Inhomogeneous_NPTBerendsen):
+    """Isotropic Berendsen NPT (ASE's ``NPTBerendsen``, dynamics.py:693-715): mu = 1 - dt beta / (3 tau_p)
+    (P0 - tr P / 3), the whole cell times mu, so its shape is kept."""
+
+    barostat = "isotropic"
+
+    def __init__(self, atoms, calculator, timestep: float = 2.0, temperature: float = 300.0, pressure: float = 1.01325e-4,
+                 taut: float | None = None, taup: float | None = None, bulk_modulus: float | None = None,
+                 fix_com: bool = True, task: PredTask | None = None) -> None:
+        super().__init__(atoms, calculator, timestep=timestep, temperature=temperature, pressure=pressure, taut=taut, taup=taup,
+                         bulk_modulus=bulk_modulus, fix_com=fix_com, task=task)
+
+    def mu(self) -> np.ndarray:
+        return np.full(3, 1.0 - self.taupscl * (self.target_pressure - self.pressure_components().sum() / 3.0))
+
+    def scale_cell(self) -> None:
+        self.atoms.set_cell(self.mu()[0] * self.atoms.cell, scale_atoms=True)
 
 
 def fire_relax(atoms, calculator: CHGNetCalculator, fmax: float = 0.1, steps: int = 500, dt: float = 0.1,

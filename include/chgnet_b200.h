@@ -340,6 +340,31 @@ int chg_md_kick(double* v, const double* f, const double* inv_mass, int32_t n_at
 int chg_fire_step(double* x, double* v, const double* f, int32_t n_atoms, double* state, const double* inv_lattice,
                   double* frac64, float* frac32, double dt_max, double max_step, void* stream);
 
+/* ---- Berendsen NVT / NPT with the cell in device memory (csrc/md.cu).  Replaces ASE's NVTBerendsen,
+ * Inhomogeneous_NPTBerendsen and NPTBerendsen that the reference's MolecularDynamics drives on the host
+ * (dynamics.py:595-609, 671-715; one CHGNetCalculator.calculate per step, dynamics.py:129-181).  Everything a
+ * captured step reads is device memory, so one CUDA graph serves every step until the lists are rebuilt.
+ * cell_state: 64 doubles = L [0..8] (rows = lattice vectors), L^-1 [9..17], L_old^-1 [18..26], L_ref [27..35] and
+ * L_ref^-1 [36..44] (the cell of the last list build), V [45], lambda [46], T [47], max_i |(s_i - s_ref,i) L_ref|^2
+ * [52], ||L_ref^-1 L - I||_F [53].  params: 8 doubles = T0 (K), P0 (eV/A^3), dt/tau_t, dt beta/(3 tau_p), mask [3],
+ * k_B (eV/K).  flags: 1 thermostat, 2 isotropic barostat, 4 per-axis barostat, 8 remove the mean momentum.
+ * mom_part [blocks][3], k_part [blocks][4] = per-block partials (blocks = chg_md_partial_blocks(n_atoms)), summed
+ * in a fixed order: the trajectory does not depend on the scheduling.  virial [9] fp64 (chg_forward's output;
+ * sigma = virial / V); lattice32 [9] is what chg_batch.lattice points at.
+ *   chg_md_cell_step      : one block: K from k_part -> lambda -> P_a = -sigma_aa + lambda^2 K_aa / V -> mu -> L, L^-1,
+ *                           V, lattice32, strain; resets the displacement maximum
+ *   chg_md_kick_drift_cell: v *= lambda; x = (x L_old^-1) L (barostat); v += dt/2 f/m; v -= mean(m v)/m (flag 8);
+ *                           x += dt v; frac64 / frac32 = x L^-1; displacement maximum against s_ref (may be NULL)
+ *   chg_md_kick_partials  : v += dt/2 f/m (f may be NULL: no kick); k_part = partials of K_aa = sum m v_a^2 and K_tr */
+int chg_md_partial_blocks(int32_t n_atoms);
+int chg_md_cell_step(const double* params, double* cell_state, const double* k_part, int32_t n_atoms,
+                     const double* virial, float* lattice32, int32_t flags, void* stream);
+int chg_md_kick_drift_cell(double* x, double* v, const double* f, const double* inv_mass, int32_t n_atoms, double dt,
+                           double* cell_state, double* mom_part, double* frac64, float* frac32, const double* s_ref,
+                           int32_t flags, void* stream);
+int chg_md_kick_partials(double* v, const double* f, const double* inv_mass, int32_t n_atoms, double dt,
+                         double* k_part, void* stream);
+
 /* ---- device CSR build: the segment structures of chg_batch from the packed index arrays
  * (replaces the torch sorts / searchsorted / nonzero of BatchedGraph-side preprocessing; csrc/batch_csr.cu).
  * Inputs: directed edges sorted by centre, angles sorted by bond i (chg_pack_batch_host reports both).
